@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Vista denoising hot path on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config full|small]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config full|small] [--dump-outputs DIR]
 
 A bench "step" is ONE EDM/Euler sampler step of a 25-frame 576x1024 clip: sampler_prepare ->
 UNet forward on the CFG-doubled batch (50 x 8 x 72 x 128) -> sampler_update — the loop body of
@@ -17,6 +17,11 @@ all-gather, the GroupNorm-sum all-reduce, the one-frame halos and the CFG pair e
 value = 25 frames / max-over-ranks time of the same job.  In that mode the line also carries `parity_rel_l2`: the sharded
 K-step latent against the unsharded runtime on rank 0 (exit code 4 above 3e-3).  `e2e` is the second call of the public
 engine.sample() -> decode_first_stage() pair (the first, which captures the 50-step graph, is `first_call_seconds`).
+
+--dump-outputs DIR writes, as float32 DIR/<name>.npy, what the timed calls handed back: `latent` (the latent after the
+last timed sampler step, whole), `decoded` (the timed decode_first_stage) and `e2e_frames` (the frames of the timed e2e
+call).  An output above DUMP_MAX_ELEMS elements is stored as a fixed seeded sample of that many elements (the same
+positions in every run), so that two builds can be compared output for output; weights and inputs are seeded.
 """
 from __future__ import annotations
 
@@ -36,6 +41,18 @@ sys.path.insert(0, ROOT)
 
 F_STEP_TFLOP = 153.9          # algorithmic TFLOP per EDM step at B=50, 72x128 (SURVEY.md §8d / BASELINE.md §2)
 F_DEC_CHUNK_TFLOP = 97.202    # per 14-frame VideoDecoder call
+DUMP_MAX_ELEMS = 1 << 22      # per dumped output (16 MB of float32); three outputs stay under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Writes every tensor of `arrays` as float32 <path>/<name>.npy; a larger one as a seeded sample of its elements."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float().cpu()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            t = t.flatten()[idx]
+        np.save(os.path.join(path, name + ".npy"), t.numpy())
 
 
 def load_peaks():
@@ -238,6 +255,9 @@ def run_ours(args):
     dt = e0.elapsed_time(e1) / 1e3
     clk = clocks.stop()
     finite = bool(torch.isfinite(st.x).all())
+    if args.dump_outputs:          # before the profiled step below, which advances st.x once more
+        from vista_b200.sharded import gather_latent
+        latent_out = (st.x if Tl == T else gather_latent(st.x, T, group=rt.group)).cpu()
 
     # ---- per-family breakdown of one extra eager step (CUDA events per launch; N > 1: this rank's share, with the
     #      host-side collectives bracketed as family "nccl")
@@ -262,14 +282,14 @@ def run_ours(args):
                 f.write(f"| {k} | {d} | {v['launches']} | {v['ms']:.2f} | {v['tflops']:.0f} | {v['gbs']:.0f} |\n")
 
     # ---- decode: the engine's own chunked decode_first_stage of the 25 latents (N > 1: chunks dealt out over the ranks)
-    zlat = (torch.randn(T, 4, h, w, device=dev) * 0.9)
+    zlat = (torch.randn(T, 4, h, w, device=dev, generator=torch.Generator(device=dev).manual_seed(5)) * 0.9)
     if world > 1:
         torch.distributed.broadcast(zlat, src=0)
     eng.decode_first_stage(zlat)
     torch.cuda.synchronize()
     d0, d1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     d0.record()
-    eng.decode_first_stage(zlat)
+    decoded = eng.decode_first_stage(zlat)
     d1.record()
     torch.cuda.synchronize()
     decode_s = d0.elapsed_time(d1) / 1e3
@@ -397,6 +417,8 @@ def run_ours(args):
         out["cpu_baseline"] = cpu_baseline(args.cpu_seconds)
     if rank == 0:
         print(json.dumps(out))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"latent": latent_out, "decoded": decoded, "e2e_frames": res})
     bad_parity = parity is not None and not (parity < 3e-3)
     if world > 1:
         # The measurement is complete and printed.  Leave without the NCCL / interpreter teardown: a multi-rank process
@@ -538,13 +560,7 @@ def run_reference(args):
         return
     threads, calib = pick_cpu_threads()
     h, w = 16, 32
-    times, spent, t_start = [], 0.0, time.perf_counter()
-    for i in range(args.warmup + args.steps):
-        t = cpu_sample_step(h, w, threads)
-        if i >= args.warmup or (time.perf_counter() - t_start) > 45:     # bounded warm-up on slow hosts
-            times.append(t)
-        if (time.perf_counter() - t_start) > 150 and times:               # whole arm within a few minutes
-            break
+    times = [cpu_sample_step(h, w, threads) for _ in range(args.warmup + args.steps)][args.warmup:]
     t = float(np.mean(times))
     scale = flops_scale(h, w)
     v = 25.0 / (50 * t * scale)
@@ -574,7 +590,11 @@ def main():
     ap.add_argument("--no-eager", action="store_true", help="skip the eager-GPU (oracle on cuda) denominator")
     ap.add_argument("--breakdown", default="", help="write rank 0's per-family / per-shape step breakdown (markdown) here")
     ap.add_argument("--cpu-seconds", type=float, default=20.0)
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the outputs of the timed calls as float32 DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 1 if args.impl == "reference" else 3)
     if int(os.environ.get("WORLD_SIZE", 1)) > 1:
         # multi-rank watchdog: a rank that is still here after 15 minutes is stuck in a collective; exit non-zero

@@ -316,9 +316,20 @@ def gen_full_step():
                         cpu_seconds=dt, cpu_threads=torch.get_num_threads())
 
 
+def gen_seam():
+    """Control runs of tests/test_reference_seam_cpu.py: the reference's own sample_utils.do_sample and
+    reward_utils.do_sample on the all-reference engine at tiny sizes, their random draws replaced by seeded tensors."""
+    sys.path.insert(0, os.path.dirname(GOLDEN_DIR))
+    import test_reference_seam_cpu as seam
+    t0 = time.time()
+    for name, arrays in seam.control_runs().items():
+        print(f"{name}: {sorted(arrays)} ({time.time() - t0:.0f}s)")
+        np.savez_compressed(os.path.join(GOLDEN_DIR, name + ".npz"), **arrays)
+
+
 def main(argv):
     os.makedirs(GOLDEN_DIR, exist_ok=True)
-    cases = argv or (["anchors"] + list(UNET_CASES) + list(SAMPLER_CASES) + list(DECODER_CASES) + list(DECODE_FS_CASES) + list(ENCODER_CASES) + ["cond_embedder_tiny"])
+    cases = argv or (["anchors"] + list(UNET_CASES) + list(SAMPLER_CASES) + list(DECODER_CASES) + list(DECODE_FS_CASES) + list(ENCODER_CASES) + ["cond_embedder_tiny", "seam"])
     for cname in cases:
         if cname == "anchors":
             gen_anchors()
@@ -336,6 +347,8 @@ def main(argv):
             gen_encoder(cname)
         elif cname == "cond_embedder_tiny":
             gen_cond_embedder(cname)
+        elif cname == "seam":
+            gen_seam()
         elif cname == "vista_full_step":
             gen_full_step()
         else:
