@@ -226,7 +226,10 @@ def test_gemm_temporal_conv_with_halo_frames(ops, nb, T, S, Cc):
                                               (2, 300, 1),
                                               # more work items than SMs (persistent loop of v5: 200 / 200 items), with and
                                               # without a skipped second query tile in the last block of a (frame, head)
-                                              (10, 1280, 4), (20, 320, 5)])
+                                              (10, 1280, 4), (20, 320, 5),
+                                              # level 0 of the full-size network (72 x 128 tokens) and the inner levels
+                                              # of the tiny / small networks (sequences below one 128-row tile)
+                                              (2, 9216, 5), (2, 32, 2), (3, 8, 1)])
 def test_attention_spatial(ops, frames, seq, heads, impl):
     Cc = heads * 64
     qkv = rnd(frames * seq, 3 * Cc, seed=23)
@@ -234,8 +237,30 @@ def test_attention_spatial(ops, frames, seq, heads, impl):
     ops.attention_spatial(qkv[:, :Cc], qkv[:, Cc:2 * Cc], qkv[:, 2 * Cc:], out, frames, seq, heads, impl=impl)
     torch.cuda.synchronize()
     q, k, v = (t.float().reshape(frames, seq, heads, 64).permute(0, 2, 1, 3) for t in qkv.chunk(3, dim=-1))
+    if seq <= 4096:
+        ref = F.scaled_dot_product_attention(q, k, v).permute(0, 2, 1, 3).reshape(frames * seq, Cc)
+        check(out, ref, rtol=4e-3, atol=2e-3, name="attn spatial")
+        return
+    # long sequences: fp64 reference of a fixed random subset of 512 query rows (the same rows in every frame and head)
+    rows = torch.randperm(seq, generator=torch.Generator().manual_seed(5))[:512].to(dev())
+    ref = F.scaled_dot_product_attention(q[:, :, rows].double(), k.double(), v.double())     # frames, heads, 512, 64
+    got = out.reshape(frames, seq, heads, 64)[:, rows].permute(0, 2, 1, 3)
+    check(got, ref, rtol=4e-3, atol=2e-3, name="attn spatial (row subset)")
+
+
+@pytest.mark.parametrize("impl", ATTN_IMPLS)
+def test_attention_spatial_strided_out(ops, impl):
+    """out is a column slice of a wider buffer (ld_o > C); the columns around it stay untouched."""
+    frames, seq, heads = 2, 300, 2
+    Cc = heads * 64
+    qkv = rnd(frames * seq, 3 * Cc, seed=27)
+    obuf = torch.full((frames * seq, Cc + 64), 7.0, dtype=torch.float16, device=dev())
+    ops.attention_spatial(qkv[:, :Cc], qkv[:, Cc:2 * Cc], qkv[:, 2 * Cc:], obuf[:, 32:32 + Cc], frames, seq, heads, impl=impl)
+    torch.cuda.synchronize()
+    q, k, v = (t.double().reshape(frames, seq, heads, 64).permute(0, 2, 1, 3) for t in qkv.chunk(3, dim=-1))
     ref = F.scaled_dot_product_attention(q, k, v).permute(0, 2, 1, 3).reshape(frames * seq, Cc)
-    check(out, ref, rtol=4e-3, atol=2e-3, name="attn spatial")
+    check(obuf[:, 32:32 + Cc], ref, rtol=4e-3, atol=2e-3, name="attn spatial strided out")
+    assert bool((obuf[:, :32] == 7.0).all()) and bool((obuf[:, 32 + Cc:] == 7.0).all())
 
 
 @pytest.mark.parametrize("impl", ATTN_IMPLS)
@@ -268,7 +293,11 @@ def test_attention_spatial_increasing_max(ops, impl):
     check(out, ref, rtol=1e-2, atol=1e-2, name="attn increasing max")
 
 
-@pytest.mark.parametrize("nb,T,S,heads", [(2, 25, 32, 1), (2, 25, 20, 5), (1, 14, 16, 2), (2, 25, 8, 20)])
+@pytest.mark.parametrize("nb,T,S,heads", [(2, 25, 32, 1), (2, 25, 20, 5), (1, 14, 16, 2), (2, 25, 8, 20),
+                                          # 23040 (clip, pixel, head) items: every warp walks several (the Q tile of
+                                          # each holds the previous item's O in its padding rows)
+                                          (2, 25, 2304, 5),
+                                          (1, 32, 64, 2), (2, 1, 40, 1), (1, 17, 96, 3)])  # no key padding, one frame, odd T
 def test_attention_temporal(ops, nb, T, S, heads):
     Cc = heads * 64
     qkv = rnd(nb * T * S, 3 * Cc, seed=25)
@@ -279,6 +308,21 @@ def test_attention_temporal(ops, nb, T, S, heads):
     ref = F.scaled_dot_product_attention(q, k, v)          # (nb, S, heads, T, 64)
     ref = ref.permute(0, 3, 1, 2, 4).reshape(nb * T * S, Cc)
     check(out, ref, name="attn temporal")
+
+
+def test_attention_temporal_peaky_strided_out(ops):
+    """Large logits (inputs x 2.5) and out as a column slice of a wider buffer."""
+    nb, T, S, heads = 2, 25, 40, 2
+    Cc = heads * 64
+    qkv = rnd(nb * T * S, 3 * Cc, seed=26, scale=2.5)
+    obuf = torch.full((nb * T * S, Cc + 64), 7.0, dtype=torch.float16, device=dev())
+    ops.attention_temporal(qkv[:, :Cc], qkv[:, Cc:2 * Cc], qkv[:, 2 * Cc:], obuf[:, 64:], nb, T, S, heads)
+    torch.cuda.synchronize()
+    q, k, v = (t.double().reshape(nb, T, S, heads, 64).permute(0, 2, 3, 1, 4) for t in qkv.chunk(3, dim=-1))
+    ref = F.scaled_dot_product_attention(q, k, v).permute(0, 3, 1, 2, 4).reshape(nb * T * S, Cc)
+    # P is rounded to fp16 before P V; with peaked rows and |v| ~ 2.5 that costs more than the 2e-3 of the plain test
+    check(obuf[:, 64:], ref, rtol=1e-2, atol=1e-2, name="attn temporal peaky")
+    assert bool((obuf[:, :64] == 7.0).all())
 
 
 # ------------------------------------------------------------------------------------------ norms
@@ -302,7 +346,7 @@ def test_groupnorm(ops, frames, tpf, Cc, fps, silu):
     check(y, ref.permute(0, 2, 1).reshape(frames * tpf, Cc), name="groupnorm")
 
 
-@pytest.mark.parametrize("tokens,Cc", [(100, 64), (1000, 320), (333, 1280), (77, 2560)])
+@pytest.mark.parametrize("tokens,Cc", [(100, 64), (1000, 320), (333, 1280), (77, 2560), (517, 640)])
 def test_layernorm(ops, tokens, Cc):
     x = rnd(tokens, Cc, seed=29, scale=1.5) - 0.3
     gamma = rnd(Cc, seed=30, dtype=torch.float32) * 0.1 + 1
@@ -316,6 +360,21 @@ def test_layernorm(ops, tokens, Cc):
     torch.cuda.synchronize()
     idx = (torch.arange(tokens, device=dev()) // 7) % 5
     check(y, F.layer_norm(x.float() + add[idx], (Cc,), gamma, beta, 1e-5), name="layernorm+add")
+
+
+@pytest.mark.parametrize("Cc", [96, 320, 640, 1280])
+def test_layernorm_strided(ops, Cc):
+    """x and y are column slices of wider buffers (ldx, ldy > C); y's neighbouring columns stay untouched."""
+    tokens = 389
+    xbuf = rnd(tokens, Cc + 40, seed=29, scale=1.5)
+    x = xbuf[:, 24:24 + Cc]
+    gamma = rnd(Cc, seed=30, dtype=torch.float32) * 0.1 + 1
+    beta = rnd(Cc, seed=31, dtype=torch.float32) * 0.1
+    ybuf = torch.full((tokens, Cc + 16), 7.0, dtype=torch.float16, device=dev())
+    ops.layernorm(x, ybuf[:, 8:8 + Cc], gamma, beta, 1e-5)
+    torch.cuda.synchronize()
+    check(ybuf[:, 8:8 + Cc], F.layer_norm(x.double(), (Cc,), gamma.double(), beta.double(), 1e-5), name="layernorm strided")
+    assert bool((ybuf[:, :8] == 7.0).all()) and bool((ybuf[:, 8 + Cc:] == 7.0).all())
 
 
 # ------------------------------------------------------------------------------------------ small ops
@@ -358,6 +417,70 @@ def test_downsample_via_im2col(ops):
     torch.cuda.synchronize()
     ref = F.conv2d(x.float().permute(0, 3, 1, 2), wt.float(), bias, stride=2, padding=1).permute(0, 2, 3, 1)
     check(out.reshape(NB, Ho, Wo, Cc), ref, name="downsample")
+
+
+@pytest.mark.parametrize("NB,H,W", [(2, 16, 24), (1, 17, 23), (3, 9, 14)])
+def test_downsample_asym_via_im2col(ops, NB, H, W):
+    """VAE-encoder Downsample: zero pad right / bottom by one, 3x3 stride 2 (even and odd H, W)."""
+    Cc = 64
+    xbuf = rnd(NB * H * W, Cc + 16, seed=54)
+    x = xbuf[:, 16:]                                      # strided input rows
+    wt = rnd(Cc, Cc, 3, 3, seed=55, scale=(9 * Cc) ** -0.5)
+    bias = rnd(Cc, seed=56, dtype=torch.float32)
+    Ho, Wo = (H - 2) // 2 + 1, (W - 2) // 2 + 1
+    col = torch.empty(NB * Ho * Wo, 9 * Cc, dtype=torch.float16, device=dev())
+    ops.im2col_s2_asym(x, col, NB, H, W, Cc)
+    out = torch.empty(NB * Ho * Wo, Cc, dtype=torch.float16, device=dev())
+    ops.gemm(col, wt.permute(0, 2, 3, 1).reshape(Cc, 9 * Cc).contiguous(), out, bias=bias)
+    torch.cuda.synchronize()
+    x4 = x.double().reshape(NB, H, W, Cc).permute(0, 3, 1, 2)
+    ref = F.conv2d(F.pad(x4, (0, 1, 0, 1)), wt.double(), bias.double(), stride=2).permute(0, 2, 3, 1)
+    check(out.reshape(NB, Ho, Wo, Cc), ref, name="downsample asym")
+
+
+@pytest.mark.parametrize("cols,ld_in", [(128, 128), (1152, 1152), (9216, 9216), (1152, 1200)])
+def test_softmax_rows(ops, cols, ld_in):
+    """Random rows, a row with one dominant score and rows of large negative scores, against fp64 softmax in fp16."""
+    rows = 37
+    g = torch.Generator().manual_seed(57)
+    x = torch.randn(rows, ld_in, generator=g) * 3
+    x[1, :] = torch.randn(ld_in, generator=g)
+    x[1, cols // 3] = 60.0                               # one dominant score
+    x[2, :] = -1e4 + torch.randn(ld_in, generator=g)      # large negative scores
+    x[3, :] = -80.0 + 0.5 * torch.randn(ld_in, generator=g)
+    x = x.to(dev())
+    y = torch.full((rows, cols + 8), 7.0, dtype=torch.float16, device=dev())
+    ops.softmax_rows(x[:, :cols], y[:, :cols])
+    torch.cuda.synchronize()
+    ref = torch.softmax(x[:, :cols].double(), dim=-1).half()
+    check(y[:, :cols], ref, rtol=2e-3, atol=1e-5, name="softmax rows")
+    assert bool((y[:, cols:] == 7.0).all())
+
+
+def test_time_mix_small_skip_frames(ops):
+    """The decoder's 3 -> 3 channel (3,1,1) convolution with skipped leading frames, an output frame offset, strided
+    input rows and the chunk-overlap blend, against fp64 conv3d and fake_ops.time_mix_small."""
+    import fake_ops
+    T, h, w, Cc, skip, f0 = 6, 5, 7, 3, 2, 3
+    HW = h * w
+    xbuf = rnd(T * HW, 8, seed=58, dtype=torch.float32)
+    x = xbuf[:, :Cc]                                      # ldx = 8
+    wt = rnd(Cc, Cc, 3, seed=59, dtype=torch.float32, scale=0.5)
+    bias = rnd(Cc, seed=60, dtype=torch.float32)
+    blend = torch.tensor([0, 0, 0, 1, 0, 1], dtype=torch.int32, device=dev())
+    out0 = rnd(f0 + T + 1, Cc, h, w, seed=61, dtype=torch.float32)
+    out = out0.clone()
+    ops.time_mix_small(x, wt, bias, out, blend, T, HW, Cc, out_frame0=f0, skip_frames=skip)
+    torch.cuda.synchronize()
+    x5 = x.double().reshape(T, h, w, Cc).permute(3, 0, 1, 2)[None]               # 1, C, T, h, w
+    conv = F.conv3d(x5, wt.double()[:, :, :, None, None], bias.double(), padding=(1, 0, 0))[0].permute(1, 0, 2, 3)
+    ref = out0.double().clone()
+    for t in range(skip, T):
+        ref[f0 + t] = 0.5 * (out0[f0 + t].double() + conv[t]) if int(blend[t]) else conv[t]
+    check(out, ref, rtol=1e-5, atol=1e-5, name="time_mix_small")
+    fake = out0.cpu().clone()
+    fake_ops.time_mix_small(x.cpu(), wt.cpu(), bias.cpu(), fake, blend.cpu(), T, HW, Cc, f0, skip)
+    check(out, fake.to(dev()), rtol=1e-5, atol=1e-5, name="time_mix_small vs fake_ops")
 
 
 def test_upsample2x(ops):
